@@ -3,7 +3,7 @@
 768x432, 10 000 points per iteration) on N B200s of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--precision tc|fp32]
-                    [--workload atlas|raft|stage2|seg]
+                    [--workload atlas|raft|stage2|seg] [--dump-outputs DIR]
 
 One "step" = one loop trip of src/stage1_neural_atlas.py:151-231 (sampling, 7 mapping + 3 atlas
 evaluations, 4 losses, backward, Adam).  Prints ONE JSON line on rank 0.  Keys beyond the driver's
@@ -229,7 +229,16 @@ def main():
     ap.add_argument("--emulate-world", type=int, default=0,
                     help="profiling aid: ONE process does the work of rank 0 of an N-GPU run (frame shard 0, no "
                          "collective), so that ncu can list the per-rank kernels of the sharded step")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (the loss vector and the "
+                         "updated parameters, float32) as DIR/losses.npy and DIR/params.npy; the inputs depend only "
+                         "on the arguments, so two builds can be compared output for output (the step sums with fp32 "
+                         "atomics: two runs of one build agree to summation order, not bit for bit)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload != "atlas" or args.impl != "b200"):
+        ap.error("--dump-outputs is implemented for --workload atlas --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -319,6 +328,7 @@ def main():
                    "without (i > 5000)": {"steps": K - n_with, "it_per_s": (K - n_with) / (mid.elapsed_time(stop) / 1000.0)},
                    "note": "this rank's device time; the headline value is all K steps"}
     losses_last = trainer.losses.cpu().numpy().copy()
+    params_last = trainer.params.cpu().numpy().copy() if args.dump_outputs else None
     if world > 1:
         tms = torch.tensor([ms], device=dev)
         dist.all_reduce(tms, op=dist.ReduceOp.MAX)
@@ -445,6 +455,10 @@ def main():
                                "kind": "oracle port (the reference's torch ops) with the networks on this GPU and "
                                        "the video tensors on the host, as src/stage1_neural_atlas.py keeps them",
                                "speedup_e2e": e2e_val / (done / secs)}
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "losses.npy"), losses_last.astype(np.float32))
+            np.save(os.path.join(args.dump_outputs, "params.npy"), params_last.astype(np.float32))
         print(json.dumps(line), flush=True)
     if world > 1:
         # orderly teardown: every rank is past its last collective; drop the captured graphs (they hold NCCL

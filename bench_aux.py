@@ -249,7 +249,7 @@ def seg_line(args, rank, world, local):
     tr = SG.SegTrainer(vid, SG.pack_mask_frames(masks, dev), None, precision=prec, device=dev)
     torch.manual_seed(0)
     tr.init_like_reference()
-    steps, warm = max(2, args.steps), max(3, args.warmup)
+    steps, warm = args.steps, max(3, args.warmup)
     g = torch.Generator().manual_seed(1)
     inds_d = [torch.randint(H * W * T, (B,), generator=g).to(dev) for _ in range(8)]
     inds_h = [torch.randint(H * W * T, (B, 1), generator=g) for _ in range(8)]
@@ -301,7 +301,7 @@ def driver_line(args, rank, world, local):
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     K.set_conv_precision("tc")
-    steps, warm = max(1, min(args.steps, 20)), max(1, min(args.warmup, 3))
+    steps, warm = args.steps, max(1, min(args.warmup, 3))
     g = torch.Generator().manual_seed(rank)
     peaks, how = _peaks()
     peak_tf = float(peaks.get("bf16_tflops_sustained", peaks.get("bf16_tflops")))
