@@ -17,10 +17,6 @@ void set_error(const char* fmt, ...) {
   va_end(ap);
 }
 
-static thread_local bool g_persistent_ws = false;
-PersistentWorkspaceScope::PersistentWorkspaceScope() : prev(g_persistent_ws) { g_persistent_ws = true; }
-PersistentWorkspaceScope::~PersistentWorkspaceScope() { g_persistent_ws = prev; }
-
 static long long g_launches = 0;
 void count_launch() { ++g_launches; }
 
@@ -176,35 +172,21 @@ int64_t b200_mlp_layout(const B200MlpDesc* d, int64_t* w_off, int64_t* b_off) {
   return s.total;
 }
 
-// which of the two stage-1 architectures a descriptor is (tensor-core kernels are specialised to them): 1 mapping,
-// 2 atlas, 0 neither
-static int tc_architecture(const MlpShape& s) {
-  if (s.hidden != 256) return 0;
-  if ((s.L == 6 || s.L == 4) && s.pe == 0 && s.in_dim == 3 && s.out_dim == 2) {     // 6: the stage-1 scripts' mapping; 4: the
-    // background mapping of the segmentation variant (same kernels, two hidden 256x256 layers instead of four)
-    for (int l = 1; l < s.L; ++l) if (s.skip[l]) return 0;
-    return 1;
-  }
-  if (s.L == 8 && s.pe == 10 && s.in_dim == 2 && s.out_dim == 3) {
-    for (int l = 1; l < s.L; ++l) if (s.skip[l] != (l == 4 || l == 7)) return 0;
-    return 2;
-  }
-  if (s.L == 8 && s.pe == 5 && s.in_dim == 3 && s.out_dim == 1) {      // alpha network of the segmentation variant
-    for (int l = 1; l < s.L; ++l) if (s.skip[l]) return 0;
-    return 3;
-  }
-  return 0;
-}
-
+// the tensor-core family of a descriptor as its ABI code: 1 mapping (6 or 4 layers), 2 atlas, 3 alpha, 0 none
 int b200_mlp_tc_architecture(const B200MlpDesc* d) {
   MlpShape s;
   if (resolve_mlp(d, &s) != B200_OK) return -1;
-  return tc_architecture(s);
+  switch (tc_classify(s)) {
+    case TcNet::Mapping6: case TcNet::Mapping4: return 1;
+    case TcNet::Atlas: return 2;
+    case TcNet::Alpha: return 3;
+    default: return 0;
+  }
 }
 
 // buffers of a stand-alone tensor-core call, carved from the caller's workspace
 struct TcCallPlan { int* gmax2; float* x; float* y; float* dy; float* d_in; char* tc; int64_t bytes; };
-static void plan_tc_call(const MlpShape& s, int arch, int64_t rows_pad, char* base, TcCallPlan* pl) {
+static void plan_tc_call(const MlpShape& s, TcNet net, int64_t rows_pad, char* base, TcCallPlan* pl) {
   char* p = base;
   pl->gmax2 = reinterpret_cast<int*>(carve(p, 64));
   pl->x = reinterpret_cast<float*>(carve(p, rows_pad * 16));
@@ -212,7 +194,7 @@ static void plan_tc_call(const MlpShape& s, int arch, int64_t rows_pad, char* ba
   pl->dy = reinterpret_cast<float*>(carve(p, rows_pad * s.out_dim * 4));
   pl->d_in = reinterpret_cast<float*>(carve(p, rows_pad * 8));
   pl->tc = p;
-  pl->bytes = (p - base) + tc_single_workspace_bytes(s, arch >= 2, rows_pad);
+  pl->bytes = (p - base) + tc_single_workspace_bytes(s, net, rows_pad);
 }
 
 int64_t b200_mlp_workspace_bytes(const B200MlpDesc* d, int64_t rows, int training) {
@@ -220,27 +202,27 @@ int64_t b200_mlp_workspace_bytes(const B200MlpDesc* d, int64_t rows, int trainin
   if (resolve_mlp(d, &s) != B200_OK || rows < 0) return -1;
   const int64_t rows_pad = round_up(rows, kTileRows);
   int64_t need = plan_mlp_scratch(s, rows_pad, training != 0, nullptr, nullptr) + 256;
-  const int arch = tc_architecture(s);
-  if (arch) {          // enough for either precision
+  const TcNet net = tc_classify(s);
+  if (net != TcNet::None) {          // enough for either precision
     TcCallPlan pl;
-    plan_tc_call(s, arch, rows_pad, nullptr, &pl);
+    plan_tc_call(s, net, rows_pad, nullptr, &pl);
     if (pl.bytes + 2048 > need) need = pl.bytes + 2048;
   }
   return need;
 }
 
-static int tc_call_prepare(const B200MlpDesc* d, int64_t rows, void* ws, int64_t ws_bytes, MlpShape* s, int* arch,
+static int tc_call_prepare(const B200MlpDesc* d, int64_t rows, void* ws, int64_t ws_bytes, MlpShape* s, TcNet* net,
                            int64_t* rows_pad, TcCallPlan* pl) {
   B200_PROPAGATE(resolve_mlp(d, s));
-  *arch = tc_architecture(*s);
-  B200_REQUIRE(*arch != 0, "B200_PREC_TC serves the stage-1 architectures (mapping: 3-256x{2,4}-2 without encoding; alpha: 3-PE5-256x6-1; "
+  *net = tc_classify(*s);
+  B200_REQUIRE(*net != TcNet::None, "B200_PREC_TC serves the stage-1 architectures (mapping: 3-256x{2,4}-2 without encoding; alpha: 3-PE5-256x6-1; "
                "atlas: 2-PE10-256x6-3 with skips 4, 7); use B200_PREC_FP32 for other shapes");
   if (!b200_device_supports_tc()) { set_error("B200_PREC_TC needs a compute-capability 10.x device"); return B200_ERR_UNSUPPORTED; }
   B200_REQUIRE(rows > 0 && rows < (1ll << 26), "rows out of range: %lld", (long long)rows);
   B200_REQUIRE(ws != nullptr, "null workspace");
   *rows_pad = round_up(rows, kTileRows);
   char* base = reinterpret_cast<char*>(round_up(reinterpret_cast<int64_t>(ws), 1024));
-  plan_tc_call(*s, *arch, *rows_pad, base, pl);
+  plan_tc_call(*s, *net, *rows_pad, base, pl);
   if (base + pl->bytes > reinterpret_cast<char*>(ws) + ws_bytes) {
     set_error("workspace too small: need %lld bytes", (long long)(pl->bytes + 2048));
     return B200_ERR_WORKSPACE;
@@ -263,16 +245,24 @@ static int mlp_prepare(const B200MlpDesc* d, int64_t rows, void* ws, int64_t ws_
   return B200_OK;
 }
 
-int b200_mlp_forward(const B200MlpDesc* d, const float* params, const float* x, float* y, int64_t rows,
-                     int training, int precision, void* ws, int64_t ws_bytes, void* stream) {
+}  // extern "C"
+
+namespace b200 {
+
+int mlp_precision(const B200MlpDesc* d, int precision) {
+  return (precision == B200_PREC_TC && b200_mlp_tc_architecture(d) > 0) ? B200_PREC_TC : B200_PREC_FP32;
+}
+
+int mlp_forward(const B200MlpDesc* d, const float* params, const float* x, float* y, int64_t rows, int training,
+                int precision, void* ws, int64_t ws_bytes, void* stream, bool persistent) {
   MlpShape s; MlpScratch sc; RowSpan span;
   B200_REQUIRE(params && x && y, "null pointer");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   if (precision == B200_PREC_TC) {
-    int arch; int64_t rows_pad; TcCallPlan pl;
-    B200_PROPAGATE(tc_call_prepare(d, rows, ws, ws_bytes, &s, &arch, &rows_pad, &pl));
-    B200_PROPAGATE(launch_pack_rows(x, s.in_dim, s.in_dim, pl.x, arch == 2 ? 2 : 4, rows, rows_pad, st));
-    B200_PROPAGATE(tc_single_forward(s, arch >= 2, params, pl.x, pl.y, rows_pad, training != 0, pl.tc, g_persistent_ws, st));
+    TcNet net; int64_t rows_pad; TcCallPlan pl;
+    B200_PROPAGATE(tc_call_prepare(d, rows, ws, ws_bytes, &s, &net, &rows_pad, &pl));
+    B200_PROPAGATE(launch_pack_rows(x, s.in_dim, s.in_dim, pl.x, net == TcNet::Atlas ? 2 : 4, rows, rows_pad, st));
+    B200_PROPAGATE(tc_single_forward(s, net, params, pl.x, pl.y, rows_pad, training != 0, pl.tc, persistent, st));
     B200_CHECK_CUDA(cudaMemcpyAsync(y, pl.y, (size_t)rows * s.out_dim * 4, cudaMemcpyDeviceToDevice, st));
     return B200_OK;
   }
@@ -295,24 +285,24 @@ int b200_mlp_forward(const B200MlpDesc* d, const float* params, const float* x, 
   return B200_OK;
 }
 
-int b200_mlp_backward(const B200MlpDesc* d, const float* params, const float* x, const float* dy,
-                      float* dparams, float* dx, int64_t rows, int precision, void* ws, int64_t ws_bytes,
-                      void* stream) {
+int mlp_backward(const B200MlpDesc* d, const float* params, const float* x, const float* dy, float* dparams, float* dx,
+                 int64_t rows, int precision, void* ws, int64_t ws_bytes, void* stream, bool persistent) {
   MlpShape s; MlpScratch sc; RowSpan span;
   B200_REQUIRE(params && dy && dparams && x, "null pointer");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   if (precision == B200_PREC_TC) {
     // the workspace still holds the padded input, the outputs and the activation images of the forward call
-    int arch; int64_t rows_pad; TcCallPlan pl;
-    B200_PROPAGATE(tc_call_prepare(d, rows, ws, ws_bytes, &s, &arch, &rows_pad, &pl));
-    B200_REQUIRE(arch == 2 || dx == nullptr, "the tensor-core mapping / alpha networks have no input gradient (their inputs "
+    TcNet net; int64_t rows_pad; TcCallPlan pl;
+    B200_PROPAGATE(tc_call_prepare(d, rows, ws, ws_bytes, &s, &net, &rows_pad, &pl));
+    const bool atlas = net == TcNet::Atlas;
+    B200_REQUIRE(atlas || dx == nullptr, "the tensor-core mapping / alpha networks have no input gradient (their inputs "
                  "are pixel coordinates); use B200_PREC_FP32 when x requires grad");
     B200_PROPAGATE(launch_pack_rows(dy, s.out_dim, s.out_dim, pl.dy, s.out_dim, rows, rows_pad, st));
     B200_CHECK_CUDA(cudaMemsetAsync(pl.gmax2, 0, 8, st));
-    B200_PROPAGATE(launch_absmax(pl.dy, rows_pad * s.out_dim, pl.gmax2 + (arch == 1 ? 1 : 0), st));
-    B200_PROPAGATE(tc_single_backward(s, arch >= 2, params, dparams, pl.x, pl.y, pl.dy, (arch == 2 && dx) ? pl.d_in : nullptr,
-                                      pl.gmax2, rows_pad, pl.tc, g_persistent_ws, st));
-    if (arch == 2 && dx) B200_CHECK_CUDA(cudaMemcpyAsync(dx, pl.d_in, (size_t)rows * 8, cudaMemcpyDeviceToDevice, st));
+    B200_PROPAGATE(launch_absmax(pl.dy, rows_pad * s.out_dim, pl.gmax2 + (tc_pe_kernels(net) ? 0 : 1), st));
+    B200_PROPAGATE(tc_single_backward(s, net, params, dparams, pl.x, pl.y, pl.dy, (atlas && dx) ? pl.d_in : nullptr,
+                                      pl.gmax2, rows_pad, pl.tc, persistent, st));
+    if (atlas && dx) B200_CHECK_CUDA(cudaMemcpyAsync(dx, pl.d_in, (size_t)rows * 8, cudaMemcpyDeviceToDevice, st));
     return B200_OK;
   }
   B200_REQUIRE(precision == B200_PREC_FP32, "unknown precision %d", precision);
@@ -336,6 +326,21 @@ int b200_mlp_backward(const B200MlpDesc* d, const float* params, const float* x,
     B200_PROPAGATE(simt_mlp_backward(s, params, x, s.in_dim, span, sc, dy, dparams, dx, s.in_dim, st));
   }
   return B200_OK;
+}
+
+}  // namespace b200
+
+extern "C" {
+
+int b200_mlp_forward(const B200MlpDesc* d, const float* params, const float* x, float* y, int64_t rows,
+                     int training, int precision, void* ws, int64_t ws_bytes, void* stream) {
+  return mlp_forward(d, params, x, y, rows, training, precision, ws, ws_bytes, stream, false);
+}
+
+int b200_mlp_backward(const B200MlpDesc* d, const float* params, const float* x, const float* dy,
+                      float* dparams, float* dx, int64_t rows, int precision, void* ws, int64_t ws_bytes,
+                      void* stream) {
+  return mlp_backward(d, params, x, dy, dparams, dx, rows, precision, ws, ws_bytes, stream, false);
 }
 
 int b200_video_pack(const float* frames, const float* frames_dx, const float* frames_dy, const float* flow_fwd,

@@ -6,6 +6,7 @@
 // ONE b200_mlp_forward call, then one head kernel.
 #include "atlas_internal.cuh"
 #include "loss_math.h"
+#include "tc_api.cuh"
 
 namespace b200 {
 
@@ -119,7 +120,7 @@ int b200_eval_maps(const B200MlpDesc* mapping, const float* mapping_params, cons
   eval_rows_kernel<<<(unsigned)((rp + 255) / 256), 256, 0, st>>>(*video, frame, pix_begin, count, rp, hL, hT,
                                                                   derivative_amount, pl.x3, pl.valid);
   B200_CHECK_LAUNCH();
-  const int prec = (precision == B200_PREC_TC && b200_mlp_tc_architecture(mapping) > 0) ? B200_PREC_TC : B200_PREC_FP32;
+  const int prec = mlp_precision(mapping, precision);
   B200_PROPAGATE(b200_mlp_forward(mapping, mapping_params, pl.x3, pl.uv, 4 * rp, 0, prec, pl.ws, pl.ws_bytes, stream));
   eval_head_kernel<<<(unsigned)((count + 255) / 256), 256, 0, st>>>(pl.uv, pl.valid, count, rp, (float)larger,
                                                                     uv_mapping_scale, derivative_amount,

@@ -25,7 +25,6 @@
 // Restates nn.Linear/ReLU/tanh/skip-concat forward+autograd of
 //   src/models/stage_1/implicit_neural_networks.py:62-81 for the two networks of
 //   src/stage1_neural_atlas.py:112-128.
-#include <memory>
 #include <mutex>
 #include <vector>
 
@@ -80,9 +79,9 @@ struct TcLayout { NetImages map, atl; };
 
 static char* carve_tc(char*& p, int64_t bytes) { char* r = p; p += round_up(bytes, 1024); return r; }
 
-static void plan_net(const MlpShape& s, int64_t rows, bool is_atlas, char*& p, NetImages* n) {
-  const int64_t tiles = rows / TM;
-  n->rows = rows;
+// forward weight images: per layer on tensor cores, its 64-wide k chunks (the positional-encoding part is one more)
+static void plan_fwd_images(const MlpShape& s, TcNet net, char*& p, NetImages* n) {
+  const bool is_atlas = tc_pe_kernels(net);
   int64_t off = 0;
   for (int l = 0; l < s.L; ++l) {
     int chunks = 0;
@@ -93,7 +92,14 @@ static void plan_net(const MlpShape& s, int64_t rows, bool is_atlas, char*& p, N
     off += (int64_t)chunks * 2 * STAGE_BYTES;
   }
   n->w_fwd = carve_tc(p, off);
-  off = 0;
+}
+
+static void plan_net(const MlpShape& s, int64_t rows, TcNet net, char*& p, NetImages* n) {
+  const bool is_atlas = tc_pe_kernels(net);
+  const int64_t tiles = rows / TM;
+  n->rows = rows;
+  plan_fwd_images(s, net, p, n);
+  int64_t off = 0;
   for (int l = 0; l < s.L; ++l) {
     n->w_bwd_layer[l] = off;
     const bool used = l <= s.L - 2 && (is_atlas || l >= 1);
@@ -114,8 +120,8 @@ int64_t tc_plan(const MlpShape& ms, const MlpShape& as, int64_t rows_map, int64_
                 TcPlan* out) {
   char* p = reinterpret_cast<char*>(round_up(reinterpret_cast<int64_t>(base), 1024));
   TcLayout lay{};
-  plan_net(ms, rows_map, false, p, &lay.map);
-  plan_net(as, rows_atlas, true, p, &lay.atl);
+  plan_net(ms, rows_map, TcNet::Mapping6, p, &lay.map);
+  plan_net(as, rows_atlas, TcNet::Atlas, p, &lay.atl);
   if (out) { out->base = base; out->bytes = p - base; out->rows_map = rows_map; out->rows_atlas = rows_atlas; }
   return p - base;
 }
@@ -123,8 +129,8 @@ int64_t tc_plan(const MlpShape& ms, const MlpShape& as, int64_t rows_map, int64_
 static TcLayout layout_of(const TcStep& s) {
   char* p = reinterpret_cast<char*>(round_up(reinterpret_cast<int64_t>(s.plan->base), 1024));
   TcLayout lay{};
-  plan_net(*s.ms, s.plan->rows_map, false, p, &lay.map);
-  plan_net(*s.as, s.plan->rows_atlas, true, p, &lay.atl);
+  plan_net(*s.ms, s.plan->rows_map, TcNet::Mapping6, p, &lay.map);
+  plan_net(*s.as, s.plan->rows_atlas, TcNet::Atlas, p, &lay.atl);
   return lay;
 }
 
@@ -1221,6 +1227,40 @@ static int sm_count() {
   return g_sm_count;
 }
 
+TcNet tc_classify(const MlpShape& s) {
+  if (s.hidden != HID) return TcNet::None;
+  uint32_t skips = 0;
+  for (int l = 1; l < s.L; ++l)
+    if (s.skip[l]) skips |= 1u << l;
+  if ((s.L == 6 || s.L == 4) && s.pe == 0 && s.in_dim == 3 && s.out_dim == 2 && !skips)
+    return s.L == 6 ? TcNet::Mapping6 : TcNet::Mapping4;
+  if (s.L == 8 && s.pe == 10 && s.in_dim == 2 && s.out_dim == 3 && skips == ((1u << 4) | (1u << 7))) return TcNet::Atlas;
+  if (s.L == 8 && s.pe == 5 && s.in_dim == 3 && s.out_dim == 1 && !skips) return TcNet::Alpha;
+  return TcNet::None;
+}
+
+// the fused forward / backward kernels of a network family and their dynamic shared memory
+struct TcKernels { void (*fwd)(FwdParams); void (*bwd)(BwdParams); int smem; };
+static TcKernels kernels_of(TcNet net) {
+  switch (net) {
+    case TcNet::Mapping6: return {tc_fwd_kernel<false>, tc_bwd_kernel<false>, KCfg<false>::SMEM};
+    case TcNet::Mapping4: return {tc_fwd_kernel<false, 4>, tc_bwd_kernel<false, 4>, KCfg<false>::SMEM};
+    case TcNet::Atlas: return {tc_fwd_kernel<true>, tc_bwd_kernel<true>, KCfg<true>::SMEM};
+    case TcNet::Alpha: return {tc_fwd_kernel<true, 8, 1>, tc_bwd_kernel<true, 8, 1>, KCfg<true>::SMEM};
+    default: return {nullptr, nullptr, 0};
+  }
+}
+
+// the fused kernels are persistent: at most one CTA per SM walks over the `tiles` 128-row tiles
+static void launch_fwd(TcNet net, int tiles, const FwdParams& P, cudaStream_t st) {
+  const TcKernels k = kernels_of(net);
+  k.fwd<<<min(sm_count(), tiles), TC_THREADS, k.smem, st>>>(P);
+}
+static void launch_bwd(TcNet net, int tiles, const BwdParams& P, cudaStream_t st) {
+  const TcKernels k = kernels_of(net);
+  k.bwd<<<min(sm_count(), tiles), TC_THREADS, k.smem, st>>>(P);
+}
+
 static int ensure_attrs() {
   // cudaFuncSetAttribute is per device: remember which devices of this process have been configured
   static bool done_dev[64] = {};
@@ -1229,47 +1269,14 @@ static int ensure_attrs() {
   B200_REQUIRE(dev >= 0 && dev < 64, "device ordinal %d out of range", dev);
   bool& done = done_dev[dev];
   if (done) return B200_OK;
-  B200_CHECK_CUDA(cudaFuncSetAttribute(tc_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg<false>::SMEM));
-  B200_CHECK_CUDA(cudaFuncSetAttribute(tc_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg<true>::SMEM));
-  B200_CHECK_CUDA(cudaFuncSetAttribute(tc_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg<false>::SMEM));
-  B200_CHECK_CUDA(cudaFuncSetAttribute(tc_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg<true>::SMEM));
-  B200_CHECK_CUDA(cudaFuncSetAttribute(tc_fwd_kernel<false, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg<false>::SMEM));
-  B200_CHECK_CUDA(cudaFuncSetAttribute(tc_bwd_kernel<false, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg<false>::SMEM));
-  B200_CHECK_CUDA(cudaFuncSetAttribute(tc_fwd_kernel<true, 8, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg<true>::SMEM));
-  B200_CHECK_CUDA(cudaFuncSetAttribute(tc_bwd_kernel<true, 8, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg<true>::SMEM));
+  for (TcNet net : {TcNet::Mapping6, TcNet::Mapping4, TcNet::Atlas, TcNet::Alpha}) {
+    const TcKernels k = kernels_of(net);
+    B200_CHECK_CUDA(cudaFuncSetAttribute(k.fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, k.smem));
+    B200_CHECK_CUDA(cudaFuncSetAttribute(k.bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, k.smem));
+  }
   B200_CHECK_CUDA(cudaFuncSetAttribute(tc_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, WG_SMEM));
   done = true;
   return B200_OK;
-}
-
-// Job / item tables depend only on pointers and geometry: built by one eager call per (workspace, row
-// geometry, parameter buffers), kept in device memory, reused inside captured graphs.
-struct HostTables {
-  int key_dev = -1;
-  const void* key_base = nullptr; int key_cap = 0, key_groups = 0; const void* key_params = nullptr;
-  const void* key_grads = nullptr; bool key_atlas = false; int key_flow = 0;
-  PrepJobs* d_prep = nullptr; WgradItems* d_wg = nullptr;
-  int n_wg = 0, n_prep = 0;
-};
-// Captured graphs bake a slot's device pointers in, so a slot is NEVER recycled: the list only grows (each entry
-// is ~50 KB of device memory; one entry per (device, workspace, row geometry, parameter buffers)).
-constexpr int MAX_TABLES = 4096;
-static std::vector<HostTables*> g_tabs;
-static std::mutex g_tabs_mutex;
-
-static int current_device() { int d = 0; cudaGetDevice(&d); return d; }
-
-static HostTables* find_tables(const TcStep& s) {
-  const bool atlas = s.y_atlas != nullptr;
-  const int dev = current_device();
-  std::lock_guard<std::mutex> lock(g_tabs_mutex);
-  for (size_t i = 0; i < g_tabs.size(); ++i) {
-    HostTables& t = *g_tabs[i];
-    if (t.key_dev == dev && t.key_base == s.plan->base && t.key_cap == s.cap && t.key_groups == s.n_groups && t.key_params == s.params &&
-        t.key_grads == s.grads && t.key_atlas == atlas && t.key_flow == s.flow_groups)
-      return &t;
-  }
-  return nullptr;
 }
 
 static void add_prep(PrepJobs& pj, const float* W, int ldw, int n_rows, int k0, int k_cnt, int transpose, char* dst) {
@@ -1280,12 +1287,9 @@ static void add_prep(PrepJobs& pj, const float* W, int ldw, int n_rows, int k0, 
 
 
 // ---- table builders shared by the cached (training loop) and the ephemeral (stand-alone IMLP) paths
-// the atlas network back-propagates to its input (uv) through the positional encoding; the alpha network's inputs
-// are pixel coordinates
-static bool net_has_dpe(const MlpShape& sh, bool is_atlas) { return is_atlas && sh.in_dim == 2; }
-
-static void prep_jobs_for_net(PrepJobs& pj, const MlpShape& sh, const NetImages& im, const float* pp, bool is_atlas,
+static void prep_jobs_for_net(PrepJobs& pj, const MlpShape& sh, const NetImages& im, const float* pp, TcNet net,
                               bool with_bwd) {
+  const bool is_atlas = tc_pe_kernels(net);
   for (int l = 0; l < sh.L; ++l) {
     char* dst = im.w_fwd + im.w_fwd_layer[l];
     if (im.n_chunks_fwd[l] == 0) continue;
@@ -1297,7 +1301,9 @@ static void prep_jobs_for_net(PrepJobs& pj, const MlpShape& sh, const NetImages&
   }
   if (!with_bwd) return;
   for (int l = 0; l < sh.L - 1; ++l) {
-    if (l < 1 && !net_has_dpe(sh, is_atlas)) continue;
+    // the atlas network back-propagates to its input (uv) through the positional encoding; the alpha network's inputs
+    // are pixel coordinates
+    if (l < 1 && net != TcNet::Atlas) continue;
     char* dst = im.w_bwd + im.w_bwd_layer[l];
     const float* W = pp + sh.w_off[l];
     // image rows = input index k of layer l (256, or 40 for atlas layer 0), chunk over the output index n
@@ -1317,8 +1323,9 @@ static double step_cost(int cols) { return cols >= 512 ? 512.0 : (cols >= 320 ? 
 struct WgProto { const char* a; int64_t a_term; int a_cols; const char* b; int64_t b_term; int b_cols;
                  float* out; int ld; int n_rows, n_cols, groups; double bytes; int mapping; };
 
-static void protos_for_net(WgProto* protos, int& np, const MlpShape& sh, const NetImages& im, float* g, bool is_atlas,
+static void protos_for_net(WgProto* protos, int& np, const MlpShape& sh, const NetImages& im, float* g, TcNet net,
                            int groups) {
+  const bool is_atlas = tc_pe_kernels(net);
   auto add = [&](const char* a, int64_t a_term, int a_cols, const char* b, int64_t b_term, int b_cols, float* out, int ld,
                  int n_rows, int n_cols) {
     protos[np++] = WgProto{a, a_term, a_cols, b, b_term, b_cols, out, ld, n_rows, n_cols, groups,
@@ -1383,57 +1390,110 @@ static void apportion_items(WgradItems& wi, const WgProto* protos, int np, int c
   }
 }
 
-static int build_tables(const TcStep& s, const TcLayout& lay, cudaStream_t st, HostTables** out) {
-  if (HostTables* t = find_tables(s)) { *out = t; return B200_OK; }
+// ---- job tables: PrepJobs (weight-image preparation) and WgradItems (weight-gradient work list).  They depend only on
+// pointers and geometry.  Callers that keep their workspace and parameter / gradient buffers alive across calls (the
+// fused loop, persistent stand-alone calls) have them built by one eager call into device allocations of their own and
+// reuse them afterwards, inside captured graphs too; ephemeral callers get them uploaded into their workspace on every
+// call.
+enum TableKind { TABLE_PREP, TABLE_WGRAD };
+// TableKey::nets of the fused loop (the mapping network alone in pre-training, with the atlas network in the loop); a
+// stand-alone call uses its TcNet.  It also fixes the workspace layout the table points into.
+constexpr int NETS_LOOP_MAPPING = 16, NETS_LOOP_ATLAS = 17;
+
+struct TableKey {
+  int dev; const void* ws; TableKind kind; int nets;
+  int64_t rows; int groups;      // rows per group, groups
+  const void* ptr;               // parameters (TABLE_PREP) or gradients (TABLE_WGRAD)
+  int flow_groups; bool training;
+  bool operator==(const TableKey& o) const {
+    return dev == o.dev && ws == o.ws && kind == o.kind && nets == o.nets && rows == o.rows && groups == o.groups &&
+           ptr == o.ptr && flow_groups == o.flow_groups && training == o.training;
+  }
+};
+struct TableEntry { TableKey key; void* d; int n; };
+// Captured graphs bake an entry's device pointer in, so an entry is NEVER recycled: the store only grows (up to ~60 KB
+// of device memory per entry; one entry per table kind and (device, workspace, row geometry, parameter or gradient
+// buffer)).
+constexpr int MAX_TABLES = 4096;
+static std::vector<TableEntry> g_tables;
+static std::mutex g_tables_mutex;
+
+static int current_device() { int d = 0; cudaGetDevice(&d); return d; }
+
+static bool stream_is_capturing(cudaStream_t st) {
   cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
   cudaStreamIsCapturing(st, &cs);
-  if (cs == cudaStreamCaptureStatusActive) {
-    set_error("tensor-core tables must be built by one eager call before graph capture");
-    return B200_ERR_INVALID;
+  return cs == cudaStreamCaptureStatusActive;
+}
+
+static bool find_table(const TableKey& key, void** d, int* n) {
+  std::lock_guard<std::mutex> lock(g_tables_mutex);
+  for (const TableEntry& e : g_tables)
+    if (e.key == key) { *d = e.d; *n = e.n; return true; }
+  return false;
+}
+
+static int table_capacity(const PrepJobs&) { return MAX_PREP_JOBS; }
+static int table_capacity(const WgradItems&) { return MAX_WGRAD_ITEMS; }
+
+// The table of `key` (nullptr: an ephemeral caller) in *d_out / *n_out: found in the store, or built on the host by
+// fill(table) and then kept in the store, or uploaded into `slot` in the caller's workspace when the caller is ephemeral
+// or the store is full.  Building takes an eager call (a pageable copy).
+template <class T, class Fill>
+static int get_table(const TableKey* key, T* slot, cudaStream_t st, Fill fill, const T** d_out, int* n_out) {
+  void* d = nullptr;
+  if (key && find_table(*key, &d, n_out)) { *d_out = static_cast<const T*>(d); return B200_OK; }
+  B200_REQUIRE(!stream_is_capturing(st), "tensor-core job tables are built by eager calls: run the same call once "
+               "without stream capture first (only a persistent workspace keeps them for capture)");
+  static thread_local T host;
+  host = T{};
+  fill(host);
+  B200_REQUIRE(host.n <= table_capacity(host), "table overflow");
+  *n_out = host.n;
+  bool keep = key != nullptr;
+  if (keep) {
+    std::lock_guard<std::mutex> lock(g_tables_mutex);
+    if ((int)g_tables.size() >= MAX_TABLES) {
+      B200_REQUIRE(slot, "too many distinct tensor-core workspaces in one process (%d)", MAX_TABLES);
+      keep = false;
+    }
   }
-  B200_REQUIRE(s.as->L == 8 && s.ms->L == 6 && s.as->skip[4] && s.as->skip[7] && s.as->pe == 10 && s.ms->pe == 0 &&
-               s.as->hidden == HID && s.ms->hidden == HID, "tensor-core path is specialised to the two stage-1 networks");
-  {
-    std::lock_guard<std::mutex> lock(g_tabs_mutex);
-    B200_REQUIRE((int)g_tabs.size() < MAX_TABLES, "too many distinct tensor-core workspaces in one process (%d)",
-                 MAX_TABLES);
+  if (!keep) {
+    B200_CHECK_CUDA(cudaMemcpyAsync(slot, &host, sizeof(T), cudaMemcpyHostToDevice, st));
+    *d_out = slot;
+    return B200_OK;
   }
-  std::unique_ptr<HostTables> tab_owner(new HostTables());
-  HostTables& tab = *tab_owner;
-  B200_CHECK_CUDA(cudaMalloc(&tab.d_prep, sizeof(PrepJobs)));
-  B200_CHECK_CUDA(cudaMalloc(&tab.d_wg, sizeof(WgradItems)));
-  std::unique_ptr<PrepJobs> pj_owner(new PrepJobs()); std::unique_ptr<WgradItems> wi_owner(new WgradItems());
-  PrepJobs& pj = *pj_owner; WgradItems& wi = *wi_owner;
-  pj.n = 0; wi.n = 0;
-  const bool atlas = s.y_atlas != nullptr;
-  // ---- forward / dgrad weight images (the atlas network only where it is evaluated: not in pre-training)
-  prep_jobs_for_net(pj, *s.ms, lay.map, s.params, false, true);
-  if (atlas) prep_jobs_for_net(pj, *s.as, lay.atl, s.params + s.ms->total, true, true);
-  // ---- wgrad items
-  WgProto protos[32]; int np = 0;
-  protos_for_net(protos, np, *s.ms, lay.map, s.grads, false, s.n_groups);
-  if (atlas) protos_for_net(protos, np, *s.as, lay.atl, s.grads + s.ms->total, true, 3);
-  apportion_items(wi, protos, np, s.cap, s.flow_groups);
-  if (pj.n > MAX_PREP_JOBS) { set_error("table overflow"); return B200_ERR_INVALID; }
-  B200_CHECK_CUDA(cudaMemcpyAsync(tab.d_prep, &pj, sizeof(PrepJobs), cudaMemcpyHostToDevice, st));
-  B200_CHECK_CUDA(cudaMemcpyAsync(tab.d_wg, &wi, sizeof(WgradItems), cudaMemcpyHostToDevice, st));
+  B200_CHECK_CUDA(cudaMalloc(&d, sizeof(T)));
+  B200_CHECK_CUDA(cudaMemcpyAsync(d, &host, sizeof(T), cudaMemcpyHostToDevice, st));
   B200_CHECK_CUDA(cudaStreamSynchronize(st));
-  tab.n_wg = wi.n; tab.n_prep = pj.n;
-  tab.key_base = s.plan->base; tab.key_cap = s.cap; tab.key_groups = s.n_groups; tab.key_params = s.params;
-  tab.key_grads = s.grads; tab.key_atlas = atlas; tab.key_dev = current_device(); tab.key_flow = s.flow_groups;
-  {
-    std::lock_guard<std::mutex> lock(g_tabs_mutex);
-    g_tabs.push_back(tab_owner.release());
-    *out = g_tabs.back();
-  }
+  std::lock_guard<std::mutex> lock(g_tables_mutex);
+  g_tables.push_back(TableEntry{*key, d, host.n});
+  *d_out = static_cast<const T*>(d);
   return B200_OK;
 }
 
+// Kernel parameters with the settings of the fused loop (network input x * 0.5 + 0.5, activation images stored, input
+// gradient accumulated onto the loss head's); stand-alone calls override them.
 static void fill_fwd(FwdParams& P, const MlpShape& sh, const NetImages& im, const float* x, float* y,
                      const float* params, int cap, int groups, const int* n_valid) {
   P.x = x; P.y = y; P.params = params; P.img = im; P.cap = cap; P.n_groups = groups; P.n_valid = n_valid;
-  P.in_scale = 0.5f; P.in_shift = 0.5f; P.store_images = 1; P.tanh_out = 1; P.flow_groups = 0;
+  P.in_scale = 0.5f; P.in_shift = 0.5f; P.store_images = 1; P.tanh_out = sh.tanh_out ? 1 : 0; P.flow_groups = 0;
   for (int l = 0; l < sh.L; ++l) { P.w_off[l] = sh.w_off[l]; P.b_off[l] = sh.b_off[l]; }
+}
+
+static void fill_bwd(BwdParams& P, const MlpShape& sh, const NetImages& im, const float* dy, const float* y,
+                     const float* x, float* d_in, const float* params, float* grads, int cap, int groups,
+                     const int* n_valid, int* gmax_bits) {
+  P.dy = dy; P.y = y; P.x = x; P.d_in = d_in; P.params = params; P.grads = grads; P.img = im;
+  P.cap = cap; P.n_groups = groups; P.n_valid = n_valid; P.gmax_bits = gmax_bits;
+  P.in_scale = 0.5f; P.d_in_accumulate = 1; P.tanh_out = sh.tanh_out ? 1 : 0; P.flow_groups = 0;
+  for (int l = 0; l < sh.L; ++l) { P.w_off[l] = sh.w_off[l]; P.b_off[l] = sh.b_off[l]; }
+}
+
+// tables of the fused loop: the prep table depends on the parameters, the wgrad table on the gradients
+static TableKey loop_key(const TcStep& s, TableKind kind) {
+  return TableKey{current_device(), s.plan->base, kind, s.y_atlas ? NETS_LOOP_ATLAS : NETS_LOOP_MAPPING, s.cap,
+                  s.n_groups, kind == TABLE_PREP ? static_cast<const void*>(s.params) : s.grads, s.flow_groups, true};
 }
 
 // The weight images depend only on the parameters, so their preparation runs on a side stream, forked from the
@@ -1444,9 +1504,25 @@ static SideStream g_side[64];
 
 int tc_begin_step(const TcStep& s, cudaStream_t st) {
   B200_PROPAGATE(ensure_attrs());
+  B200_REQUIRE(tc_classify(*s.ms) == TcNet::Mapping6 && tc_classify(*s.as) == TcNet::Atlas,
+               "tensor-core path is specialised to the two stage-1 networks");
   const TcLayout lay = layout_of(s);
-  HostTables* tab = nullptr;
-  B200_PROPAGATE(build_tables(s, lay, st, &tab));
+  const bool atlas = s.y_atlas != nullptr;
+  const TableKey kp = loop_key(s, TABLE_PREP), kw = loop_key(s, TABLE_WGRAD);
+  const PrepJobs* d_prep; int n_prep;
+  const WgradItems* d_wg; int n_wg;
+  // forward / dgrad weight images (the atlas network only where it is evaluated: not in pre-training)
+  B200_PROPAGATE(get_table<PrepJobs>(&kp, nullptr, st, [&](PrepJobs& pj) {
+    prep_jobs_for_net(pj, *s.ms, lay.map, s.params, TcNet::Mapping6, true);
+    if (atlas) prep_jobs_for_net(pj, *s.as, lay.atl, s.params + s.ms->total, TcNet::Atlas, true);
+  }, &d_prep, &n_prep));
+  // wgrad items, for run_backward
+  B200_PROPAGATE(get_table<WgradItems>(&kw, nullptr, st, [&](WgradItems& wi) {
+    WgProto protos[32]; int np = 0;
+    protos_for_net(protos, np, *s.ms, lay.map, s.grads, TcNet::Mapping6, s.n_groups);
+    if (atlas) protos_for_net(protos, np, *s.as, lay.atl, s.grads + s.ms->total, TcNet::Atlas, 3);
+    apportion_items(wi, protos, np, s.cap, s.flow_groups);
+  }, &d_wg, &n_wg));
   SideStream& sd = g_side[current_device()];
   if (!sd.stream) {
     B200_CHECK_CUDA(cudaStreamCreateWithFlags(&sd.stream, cudaStreamNonBlocking));
@@ -1456,7 +1532,7 @@ int tc_begin_step(const TcStep& s, cudaStream_t st) {
   B200_CHECK_CUDA(cudaEventRecord(sd.fork, st));
   B200_CHECK_CUDA(cudaStreamWaitEvent(sd.stream, sd.fork, 0));
   // weight images of both networks — every step, since Adam changed the parameters
-  tc_prep_kernel<<<tab->n_prep * 4, 128, 0, sd.stream>>>(tab->d_prep);
+  tc_prep_kernel<<<n_prep * 4, 128, 0, sd.stream>>>(d_prep);
   B200_CHECK_LAUNCH();
   B200_CHECK_CUDA(cudaEventRecord(sd.join, sd.stream));
   sd.pending = true;
@@ -1469,19 +1545,18 @@ static int run_forward(const TcStep& s, bool with_atlas, cudaStream_t st) {
   if (!sd.pending) B200_PROPAGATE(tc_begin_step(s, st));     // callers that did not fork earlier
   B200_CHECK_CUDA(cudaStreamWaitEvent(st, sd.join, 0));
   sd.pending = false;
-  const int tiles_map = s.n_groups * (s.cap / TM);
   FwdParams pm{};
   fill_fwd(pm, *s.ms, lay.map, s.x_map, s.uv, s.params, s.cap, s.n_groups, s.counters);
   pm.flow_groups = s.flow_groups;
   timer_begin(TAG_MAP_FWD, st);
-  tc_fwd_kernel<false><<<min(sm_count(), tiles_map), TC_THREADS, KCfg<false>::SMEM, st>>>(pm);
+  launch_fwd(TcNet::Mapping6, s.n_groups * (s.cap / TM), pm, st);
   timer_end(TAG_MAP_FWD, st);
   B200_CHECK_LAUNCH();
   if (with_atlas) {
     FwdParams pa{};
     fill_fwd(pa, *s.as, lay.atl, s.uv, s.y_atlas, s.params + s.ms->total, s.cap, 3, s.counters);
     timer_begin(TAG_ATLAS_FWD, st);
-    tc_fwd_kernel<true><<<min(sm_count(), 3 * (s.cap / TM)), TC_THREADS, KCfg<true>::SMEM, st>>>(pa);
+    launch_fwd(TcNet::Atlas, 3 * (s.cap / TM), pa, st);
     timer_end(TAG_ATLAS_FWD, st);
     B200_CHECK_LAUNCH();
   }
@@ -1506,35 +1581,32 @@ int tc_debug_wgrad(long long* cycles, int* shapes, int max_ctas) {
 
 static int run_backward(const TcStep& s, bool with_atlas, cudaStream_t st) {
   const TcLayout lay = layout_of(s);
-  HostTables* tab = find_tables(s);
-  if (!tab) { set_error("tensor-core backward called before forward"); return B200_ERR_INVALID; }
+  void* tab; int n_wg;
+  if (!find_table(loop_key(s, TABLE_WGRAD), &tab, &n_wg)) {
+    set_error("tensor-core backward called before forward");
+    return B200_ERR_INVALID;
+  }
+  const WgradItems* d_wg = static_cast<const WgradItems*>(tab);
   int* gmax = const_cast<int*>(s.counters) + 3;
-  auto fill = [&](BwdParams& P, const MlpShape& sh, const NetImages& im, const float* dy, const float* y,
-                  const float* x, float* d_in, const float* params, float* grads, int groups) {
-    P.dy = dy; P.y = y; P.x = x; P.d_in = d_in; P.params = params; P.grads = grads; P.img = im;
-    P.cap = s.cap; P.n_groups = groups; P.n_valid = s.counters; P.gmax_bits = gmax;
-    P.in_scale = 0.5f; P.d_in_accumulate = 1; P.tanh_out = 1; P.flow_groups = 0;
-    for (int l = 0; l < sh.L; ++l) { P.w_off[l] = sh.w_off[l]; P.b_off[l] = sh.b_off[l]; }
-  };
   if (with_atlas) {
     BwdParams pa{};
-    fill(pa, *s.as, lay.atl, s.d_y, s.y_atlas, nullptr, const_cast<float*>(s.d_uv), s.params + s.ms->total,
-         s.grads + s.ms->total, 3);
+    fill_bwd(pa, *s.as, lay.atl, s.d_y, s.y_atlas, nullptr, const_cast<float*>(s.d_uv), s.params + s.ms->total,
+             s.grads + s.ms->total, s.cap, 3, s.counters, gmax);
     timer_begin(TAG_ATLAS_BWD, st);
-    tc_bwd_kernel<true><<<min(sm_count(), 3 * (s.cap / TM)), TC_THREADS, KCfg<true>::SMEM, st>>>(pa);
+    launch_bwd(TcNet::Atlas, 3 * (s.cap / TM), pa, st);
     timer_end(TAG_ATLAS_BWD, st);
     B200_CHECK_LAUNCH();
   }
   BwdParams pm{};
-  fill(pm, *s.ms, lay.map, s.d_uv, s.uv, s.x_map, nullptr, s.params, s.grads, s.n_groups);
+  fill_bwd(pm, *s.ms, lay.map, s.d_uv, s.uv, s.x_map, nullptr, s.params, s.grads, s.cap, s.n_groups, s.counters, gmax);
   pm.flow_groups = s.flow_groups;
   timer_begin(TAG_MAP_BWD, st);
-  tc_bwd_kernel<false><<<min(sm_count(), s.n_groups * (s.cap / TM)), TC_THREADS, KCfg<false>::SMEM, st>>>(pm);
+  launch_bwd(TcNet::Mapping6, s.n_groups * (s.cap / TM), pm, st);
   timer_end(TAG_MAP_BWD, st);
   B200_CHECK_LAUNCH();
   timer_begin(TAG_WGRAD, st);
-  g_last_wg = tab->d_wg; g_last_wg_n = min(tab->n_wg, sm_count());
-  tc_wgrad_kernel<<<min(tab->n_wg, sm_count()), WG_THREADS, WG_SMEM, st>>>(tab->d_wg, s.counters, gmax);
+  g_last_wg = d_wg; g_last_wg_n = min(n_wg, sm_count());
+  tc_wgrad_kernel<<<min(n_wg, sm_count()), WG_THREADS, WG_SMEM, st>>>(d_wg, s.counters, gmax);
   timer_end(TAG_WGRAD, st);
   B200_CHECK_LAUNCH();
   return B200_OK;
@@ -1550,21 +1622,10 @@ static void plan_infer(const MlpShape& ms, const MlpShape& as, char* base, NetIm
                        PrepJobs** d_prep, int64_t* bytes) {
   char* p = reinterpret_cast<char*>(round_up(reinterpret_cast<int64_t>(base), 1024));
   *d_prep = reinterpret_cast<PrepJobs*>(carve_tc(p, sizeof(PrepJobs)));
-  for (int net = 0; net < 2; ++net) {
-    const MlpShape& s = net ? as : ms;
-    NetImages* n = net ? im_atl : im_map;
-    *n = NetImages{};
-    int64_t off = 0;
-    for (int l = 0; l < s.L; ++l) {
-      int chunks = 0;
-      const bool tc_layer = net ? (l <= s.L - 2) : (l >= 1 && l <= s.L - 2);
-      if (tc_layer) chunks = (l == 0 ? 0 : HID / 64) + ((l == 0 || s.skip[l]) && net ? 1 : 0);
-      n->n_chunks_fwd[l] = chunks;
-      n->w_fwd_layer[l] = off;
-      off += (int64_t)chunks * 2 * STAGE_BYTES;
-    }
-    n->w_fwd = carve_tc(p, off);
-  }
+  *im_map = NetImages{};
+  plan_fwd_images(ms, TcNet::Mapping6, p, im_map);
+  *im_atl = NetImages{};
+  plan_fwd_images(as, TcNet::Atlas, p, im_atl);
   *bytes = p - base;
 }
 
@@ -1577,194 +1638,105 @@ int64_t tc_infer_workspace_bytes(const MlpShape& ms, const MlpShape& as) {
 int tc_infer_forward(const MlpShape& ms, const MlpShape& as, const float* params, const float* x_map, float* uv,
                      float* y, int64_t rows, char* ws, cudaStream_t st) {
   B200_PROPAGATE(ensure_attrs());
-  B200_REQUIRE(as.L == 8 && ms.L == 6 && as.skip[4] && as.skip[7] && as.pe == 10 && ms.pe == 0 && as.hidden == HID &&
-               ms.hidden == HID, "tensor-core path is specialised to the two stage-1 networks");
+  B200_REQUIRE(tc_classify(ms) == TcNet::Mapping6 && tc_classify(as) == TcNet::Atlas,
+               "tensor-core path is specialised to the two stage-1 networks");
   B200_REQUIRE(rows > 0 && rows % TM == 0 && rows / TM < (1 << 24), "rows must be a positive multiple of %d", TM);
-  NetImages im_map, im_atl; PrepJobs* d_prep; int64_t bytes;
-  plan_infer(ms, as, ws, &im_map, &im_atl, &d_prep, &bytes);
+  NetImages im_map, im_atl; PrepJobs* slot; int64_t bytes;
+  plan_infer(ms, as, ws, &im_map, &im_atl, &slot, &bytes);
   // The job table lives in the caller's workspace and is rebuilt on every call (4 KB, pageable copy: the call is
   // not graph-capturable, which a render does not need) — nothing is cached, so a recycled workspace is harmless.
-  {
-    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-    cudaStreamIsCapturing(st, &cs);
-    B200_REQUIRE(cs != cudaStreamCaptureStatusActive, "the tensor-core render is not graph-capturable");
-  }
-  static thread_local PrepJobs pj_host;
-  PrepJobs* pj = &pj_host;
-  pj->n = 0;
-  prep_jobs_for_net(*pj, ms, im_map, params, false, false);
-  prep_jobs_for_net(*pj, as, im_atl, params + ms.total, true, false);
-  B200_CHECK_CUDA(cudaMemcpyAsync(d_prep, pj, sizeof(PrepJobs), cudaMemcpyHostToDevice, st));
-  tc_prep_kernel<<<pj->n * 4, 128, 0, st>>>(d_prep);
+  B200_REQUIRE(!stream_is_capturing(st), "the tensor-core render is not graph-capturable");
+  const PrepJobs* d_prep; int n_prep;
+  B200_PROPAGATE(get_table(nullptr, slot, st, [&](PrepJobs& pj) {
+    prep_jobs_for_net(pj, ms, im_map, params, TcNet::Mapping6, false);
+    prep_jobs_for_net(pj, as, im_atl, params + ms.total, TcNet::Atlas, false);
+  }, &d_prep, &n_prep));
+  tc_prep_kernel<<<n_prep * 4, 128, 0, st>>>(d_prep);
   B200_CHECK_LAUNCH();
   const int tiles = (int)(rows / TM);
   FwdParams pm{};
   fill_fwd(pm, ms, im_map, x_map, uv, params, (int)rows, 1, nullptr);
   pm.store_images = 0;
-  tc_fwd_kernel<false><<<min(sm_count(), tiles), TC_THREADS, KCfg<false>::SMEM, st>>>(pm);
+  launch_fwd(TcNet::Mapping6, tiles, pm, st);
   B200_CHECK_LAUNCH();
   FwdParams pa{};
   fill_fwd(pa, as, im_atl, uv, y, params + ms.total, (int)rows, 1, nullptr);
   pa.store_images = 0;
-  tc_fwd_kernel<true><<<min(sm_count(), tiles), TC_THREADS, KCfg<true>::SMEM, st>>>(pa);
+  launch_fwd(TcNet::Atlas, tiles, pa, st);
   B200_CHECK_LAUNCH();
   return B200_OK;
 }
 
 // ---------------------------------------------------------------------------------------------
-// stand-alone evaluation of ONE of the two networks with autograd support: what the `IMLP` class needs
-// (implicit_neural_networks.py:62-81 forward + the autograd of its Linear/ReLU/tanh/skip stack).  Tables are
-// rebuilt into the caller's workspace on every call (pageable copies; not graph-capturable): no process-wide cache.
+// stand-alone evaluation of ONE network with autograd support: what the `IMLP` class needs
+// (implicit_neural_networks.py:62-81 forward + the autograd of its Linear/ReLU/tanh/skip stack).  Job tables are
+// cached for persistent callers and uploaded into the workspace on every call otherwise (see get_table).
 // Workspace: [PrepJobs][WgradItems][images of the network].
 // ---------------------------------------------------------------------------------------------
 struct SinglePlan { PrepJobs* d_prep; WgradItems* d_wg; NetImages im; int64_t bytes; };
 
-static void plan_single(const MlpShape& sh, bool is_atlas, int64_t rows, char* base, SinglePlan* out) {
+static void plan_single(const MlpShape& sh, TcNet net, int64_t rows, char* base, SinglePlan* out) {
   char* p = reinterpret_cast<char*>(round_up(reinterpret_cast<int64_t>(base), 1024));
   out->d_prep = reinterpret_cast<PrepJobs*>(carve_tc(p, sizeof(PrepJobs)));
   out->d_wg = reinterpret_cast<WgradItems*>(carve_tc(p, sizeof(WgradItems)));
-  plan_net(sh, rows, is_atlas, p, &out->im);
+  plan_net(sh, rows, net, p, &out->im);
   out->bytes = p - base;
 }
 
-int64_t tc_single_workspace_bytes(const MlpShape& sh, bool is_atlas, int64_t rows) {
+int64_t tc_single_workspace_bytes(const MlpShape& sh, TcNet net, int64_t rows) {
   SinglePlan pl;
-  plan_single(sh, is_atlas, rows, nullptr, &pl);
+  plan_single(sh, net, rows, nullptr, &pl);
   return pl.bytes + 2048;
 }
 
-static int check_single(const MlpShape& sh, bool is_atlas, int64_t rows, cudaStream_t st) {
+static int check_single(const MlpShape& sh, TcNet net, int64_t rows) {
   B200_PROPAGATE(ensure_attrs());
-  if (is_atlas) {
-    bool no_skips = true;
-    for (int l = 1; l < sh.L; ++l) no_skips = no_skips && !sh.skip[l];
-    const bool atlas = sh.L == 8 && sh.skip[4] && sh.skip[7] && sh.pe == 10 && sh.hidden == HID && sh.in_dim == 2 && sh.out_dim == 3;
-    const bool alpha = sh.L == 8 && no_skips && sh.pe == 5 && sh.hidden == HID && sh.in_dim == 3 && sh.out_dim == 1;
-    B200_REQUIRE(atlas || alpha, "tensor-core IMLP: neither the atlas (2-PE10-256x6-3, skips 4,7) nor the alpha "
-                 "(3-PE5-256x6-1) architecture");
-  }
-  else {
-    bool plain = (sh.L == 6 || sh.L == 4) && sh.pe == 0 && sh.hidden == HID && sh.in_dim == 3 && sh.out_dim == 2;
-    for (int l = 1; plain && l < sh.L; ++l) plain = !sh.skip[l];
-    B200_REQUIRE(plain, "tensor-core IMLP: not a mapping architecture (3 -> 256 x {2,4} -> 2, no encoding, no skips)");
-  }
+  B200_REQUIRE(net != TcNet::None && tc_classify(sh) == net, "tensor-core IMLP: not one of the stage-1 architectures "
+               "(mapping 3-256x{2,4}-2, atlas 2-PE10-256x6-3 with skips 4,7, alpha 3-PE5-256x6-1)");
   B200_REQUIRE(rows > 0 && rows % TM == 0 && rows / TM < (1 << 20), "rows must be a positive multiple of %d", TM);
   return B200_OK;
 }
 
-static bool stream_is_capturing(cudaStream_t st) {
-  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-  cudaStreamIsCapturing(st, &cs);
-  return cs == cudaStreamCaptureStatusActive;
-}
-
-// Job tables of stand-alone calls whose caller keeps ONE workspace and ONE set of parameter / gradient buffers alive
-// across calls (the segmentation step): like the fused loop's tables they are a pure function of pointers and geometry,
-// live in their own device allocations (never recycled) and are uploaded by the first eager call, after which the
-// calls are graph-capturable.  Ephemeral callers (the IMLP class: a fresh workspace per call) keep their tables
-// inside the workspace and upload them on every call.
-struct SingleTab {
-  int dev; const void* ws; int64_t rows; const void* params; const void* grads; bool is_atlas; int L, pe, in_dim; bool training;
-  PrepJobs* d_prep = nullptr; WgradItems* d_wg = nullptr; int n_prep = -1, n_wg = -1;
-};
-static std::vector<SingleTab*> g_single_tabs;
-
-static SingleTab* single_tab(const MlpShape& sh, bool is_atlas, const void* ws, int64_t rows, const void* params,
-                             const void* grads, bool training) {
-  const int dev = current_device();
-  std::lock_guard<std::mutex> lock(g_tabs_mutex);
-  for (SingleTab* t : g_single_tabs)
-    if (t->dev == dev && t->ws == ws && t->rows == rows && t->params == params && t->is_atlas == is_atlas && t->L == sh.L &&
-        t->pe == sh.pe && t->in_dim == sh.in_dim && t->training == training && (grads == nullptr || t->grads == nullptr || t->grads == grads)) {
-      if (grads && !t->grads) t->grads = grads;
-      return t;
-    }
-  if ((int)g_single_tabs.size() >= MAX_TABLES) return nullptr;
-  SingleTab* t = new SingleTab{dev, ws, rows, params, grads, is_atlas, sh.L, sh.pe, sh.in_dim, training};
-  g_single_tabs.push_back(t);
-  return t;
-}
-
 // x: mapping [rows][4], atlas [rows][2] (network input itself).  y: [rows][out_dim].
-int tc_single_forward(const MlpShape& sh, bool is_atlas, const float* params, const float* x, float* y, int64_t rows,
+int tc_single_forward(const MlpShape& sh, TcNet net, const float* params, const float* x, float* y, int64_t rows,
                       bool training, char* ws, bool persistent, cudaStream_t st) {
-  B200_PROPAGATE(check_single(sh, is_atlas, rows, st));
+  B200_PROPAGATE(check_single(sh, net, rows));
   SinglePlan pl;
-  plan_single(sh, is_atlas, rows, ws, &pl);
-  static thread_local PrepJobs pj;
-  PrepJobs* d_prep = pl.d_prep;
-  int n_prep = 0;
-  SingleTab* tab = persistent ? single_tab(sh, is_atlas, ws, rows, params, nullptr, training) : nullptr;
-  if (tab && tab->n_prep >= 0) {
-    d_prep = tab->d_prep; n_prep = tab->n_prep;
-  } else {
-    B200_REQUIRE(!stream_is_capturing(st), "stand-alone tensor-core IMLP call under stream capture before its job tables "
-                 "exist: run the same call once eagerly first (persistent workspaces only)");
-    pj.n = 0;
-    prep_jobs_for_net(pj, sh, pl.im, params, is_atlas, training);
-    n_prep = pj.n;
-    if (tab) {
-      B200_CHECK_CUDA(cudaMalloc(&tab->d_prep, sizeof(PrepJobs)));
-      B200_CHECK_CUDA(cudaMemcpy(tab->d_prep, &pj, sizeof(PrepJobs), cudaMemcpyHostToDevice));
-      tab->n_prep = n_prep; d_prep = tab->d_prep;
-    } else {
-      B200_CHECK_CUDA(cudaMemcpyAsync(pl.d_prep, &pj, sizeof(PrepJobs), cudaMemcpyHostToDevice, st));
-    }
-  }
+  plan_single(sh, net, rows, ws, &pl);
+  const TableKey key{current_device(), ws, TABLE_PREP, (int)net, rows, 1, params, 0, training};
+  const PrepJobs* d_prep; int n_prep;
+  B200_PROPAGATE(get_table(persistent ? &key : nullptr, pl.d_prep, st, [&](PrepJobs& pj) {
+    prep_jobs_for_net(pj, sh, pl.im, params, net, training);
+  }, &d_prep, &n_prep));
   tc_prep_kernel<<<n_prep * 4, 128, 0, st>>>(d_prep);
   B200_CHECK_LAUNCH();
   FwdParams P{};
   fill_fwd(P, sh, pl.im, x, y, params, (int)rows, 1, nullptr);
-  P.in_scale = 1.0f; P.in_shift = 0.0f; P.store_images = training ? 1 : 0; P.tanh_out = sh.tanh_out ? 1 : 0;
-  const int grid = min(sm_count(), (int)(rows / TM));
-  if (is_atlas && sh.in_dim == 3) tc_fwd_kernel<true, 8, 1><<<grid, TC_THREADS, KCfg<true>::SMEM, st>>>(P);
-  else if (is_atlas) tc_fwd_kernel<true><<<grid, TC_THREADS, KCfg<true>::SMEM, st>>>(P);
-  else if (sh.L == 4) tc_fwd_kernel<false, 4><<<grid, TC_THREADS, KCfg<false>::SMEM, st>>>(P);
-  else tc_fwd_kernel<false><<<grid, TC_THREADS, KCfg<false>::SMEM, st>>>(P);
+  P.in_scale = 1.0f; P.in_shift = 0.0f; P.store_images = training ? 1 : 0;
+  launch_fwd(net, (int)(rows / TM), P, st);
   B200_CHECK_LAUNCH();
   return B200_OK;
 }
 
 // after tc_single_forward(training) on the same workspace.  y: the saved outputs, dy [rows][out_dim] (zero in padding
 // rows), gmax: device int holding the bits of max|dy| (>= 0), d_in: atlas only, [rows][2] or null.
-int tc_single_backward(const MlpShape& sh, bool is_atlas, const float* params, float* grads, const float* x,
+int tc_single_backward(const MlpShape& sh, TcNet net, const float* params, float* grads, const float* x,
                        const float* y, const float* dy, float* d_in, int* gmax2, int64_t rows, char* ws,
                        bool persistent, cudaStream_t st) {
-  B200_PROPAGATE(check_single(sh, is_atlas, rows, st));
+  B200_PROPAGATE(check_single(sh, net, rows));
   SinglePlan pl;
-  plan_single(sh, is_atlas, rows, ws, &pl);
-  static thread_local WgradItems wi;
-  WgradItems* d_wg = pl.d_wg;
-  int n_wg = 0;
-  SingleTab* tab = persistent ? single_tab(sh, is_atlas, ws, rows, params, grads, true) : nullptr;
-  if (tab && tab->n_wg >= 0) {
-    d_wg = tab->d_wg; n_wg = tab->n_wg;
-  } else {
-    B200_REQUIRE(!stream_is_capturing(st), "stand-alone tensor-core IMLP backward under stream capture before its job "
-                 "tables exist: run the same call once eagerly first (persistent workspaces only)");
-    wi.n = 0;
+  plan_single(sh, net, rows, ws, &pl);
+  const TableKey key{current_device(), ws, TABLE_WGRAD, (int)net, rows, 1, grads, 0, true};
+  const WgradItems* d_wg; int n_wg;
+  B200_PROPAGATE(get_table(persistent ? &key : nullptr, pl.d_wg, st, [&](WgradItems& wi) {
     WgProto protos[16]; int np = 0;
-    protos_for_net(protos, np, sh, pl.im, grads, is_atlas, 1);
+    protos_for_net(protos, np, sh, pl.im, grads, net, 1);
     apportion_items(wi, protos, np, (int)rows, 0);
-    n_wg = wi.n;
-    if (tab) {
-      B200_CHECK_CUDA(cudaMalloc(&tab->d_wg, sizeof(WgradItems)));
-      B200_CHECK_CUDA(cudaMemcpy(tab->d_wg, &wi, sizeof(WgradItems), cudaMemcpyHostToDevice));
-      tab->n_wg = n_wg; d_wg = tab->d_wg;
-    } else {
-      B200_CHECK_CUDA(cudaMemcpyAsync(pl.d_wg, &wi, sizeof(WgradItems), cudaMemcpyHostToDevice, st));
-    }
-  }
+  }, &d_wg, &n_wg));
   BwdParams P{};
-  P.dy = dy; P.y = y; P.x = x; P.d_in = d_in; P.params = params; P.grads = grads; P.img = pl.im;
-  P.cap = (int)rows; P.n_groups = 1; P.n_valid = nullptr; P.gmax_bits = gmax2;      // [0] atlas scale, [1] mapping scale
-  P.in_scale = 1.0f; P.d_in_accumulate = 0; P.tanh_out = sh.tanh_out ? 1 : 0; P.flow_groups = 0;
-  for (int l = 0; l < sh.L; ++l) { P.w_off[l] = sh.w_off[l]; P.b_off[l] = sh.b_off[l]; }
-  const int grid = min(sm_count(), (int)(rows / TM));
-  if (is_atlas && sh.in_dim == 3) tc_bwd_kernel<true, 8, 1><<<grid, TC_THREADS, KCfg<true>::SMEM, st>>>(P);
-  else if (is_atlas) tc_bwd_kernel<true><<<grid, TC_THREADS, KCfg<true>::SMEM, st>>>(P);
-  else if (sh.L == 4) tc_bwd_kernel<false, 4><<<grid, TC_THREADS, KCfg<false>::SMEM, st>>>(P);
-  else tc_bwd_kernel<false><<<grid, TC_THREADS, KCfg<false>::SMEM, st>>>(P);
+  fill_bwd(P, sh, pl.im, dy, y, x, d_in, params, grads, (int)rows, 1, nullptr, gmax2);   // [0] atlas scale, [1] mapping scale
+  P.in_scale = 1.0f; P.d_in_accumulate = 0;
+  launch_bwd(net, (int)(rows / TM), P, st);
   B200_CHECK_LAUNCH();
   tc_wgrad_kernel<<<min(n_wg, sm_count()), WG_THREADS, WG_SMEM, st>>>(d_wg, nullptr, gmax2);
   B200_CHECK_LAUNCH();

@@ -60,8 +60,7 @@ static int plan_seg(const B200SegConfig* cfg, char* base, SegPlan* pl) {
     B200_PROPAGATE(resolve_mlp(descs[k], &pl->net[k].s));
     pl->net[k].p_off = off;
     off += pl->net[k].s.total;
-    const int arch = b200_mlp_tc_architecture(descs[k]);
-    pl->net[k].prec = (cfg->precision == B200_PREC_TC && arch > 0) ? B200_PREC_TC : B200_PREC_FP32;
+    pl->net[k].prec = mlp_precision(descs[k], cfg->precision);
   }
   pl->total_params = off;
   const MlpShape& m1 = pl->net[0].s; const MlpShape& m2 = pl->net[1].s;
@@ -327,7 +326,6 @@ int b200_seg_loss_grad(const B200SegConfig* cfg, const B200Video* video, const f
   B200_PROPAGATE(seg_prepare(cfg, ws, ws_bytes, &pl));
   // the caller keeps `ws`, `params` and `grads` across trips: the networks' job tables are cached after the first
   // (eager) trip, which also makes the whole trip graph-capturable
-  PersistentWorkspaceScope persistent;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const int cap = pl.cap, B = cfg->batch;
   const B200MlpDesc* descs[4] = {&cfg->mapping1, &cfg->mapping2, &cfg->alpha, &cfg->atlas};
@@ -353,13 +351,13 @@ int b200_seg_loss_grad(const B200SegConfig* cfg, const B200Video* video, const f
   float* const douts[4] = {pl.d_uv1, pl.d_uv2, pl.d_ar, pl.d_yat};
   const int64_t net_rows[4] = {map_rows, map_rows, (int64_t)A_COUNT * cap, (int64_t)SEG_ATLAS_ROWS * cap};
   for (int k = 0; k < 3; ++k)
-    B200_PROPAGATE(b200_mlp_forward(descs[k], params + pl.net[k].p_off, ins[k], outs[k], net_rows[k], 1,
-                                    pl.net[k].prec, pl.net[k].ws, pl.net[k].ws_bytes, stream));
+    B200_PROPAGATE(mlp_forward(descs[k], params + pl.net[k].p_off, ins[k], outs[k], net_rows[k], 1, pl.net[k].prec,
+                               pl.net[k].ws, pl.net[k].ws_bytes, stream, true));
   const int64_t layer_rows = 3ll * cap;
   seg_atlas_in_kernel<<<(unsigned)((2 * layer_rows + 255) / 256), 256, 0, st>>>(pl.uv1, pl.uv2, layer_rows, pl.xat);
   B200_CHECK_LAUNCH();
-  B200_PROPAGATE(b200_mlp_forward(descs[3], params + pl.net[3].p_off, pl.xat, pl.yat, (int64_t)SEG_ATLAS_ROWS * cap, 1,
-                                  pl.net[3].prec, pl.net[3].ws, pl.net[3].ws_bytes, stream));
+  B200_PROPAGATE(mlp_forward(descs[3], params + pl.net[3].p_off, pl.xat, pl.yat, (int64_t)SEG_ATLAS_ROWS * cap, 1,
+                             pl.net[3].prec, pl.net[3].ws, pl.net[3].ws_bytes, stream, true));
   SegLossConfig lc;
   lc.larger_dim = (float)larger; lc.uv_scale = cfg->uv_mapping_scale;
   lc.d_local = cfg->derivative_amount; lc.d_global = cfg->global_derivative_amount;
@@ -372,13 +370,13 @@ int b200_seg_loss_grad(const B200SegConfig* cfg, const B200Video* video, const f
                                                       cap, B, lc, pl.d_uv1, pl.d_uv2, pl.d_ar, pl.d_yat, losses);
   B200_CHECK_LAUNCH();
   // backward: atlas first (its input gradient feeds both mappings), then the other three networks
-  B200_PROPAGATE(b200_mlp_backward(descs[3], params + pl.net[3].p_off, pl.xat, pl.d_yat, grads + pl.net[3].p_off, pl.d_xat,
-                                   (int64_t)SEG_ATLAS_ROWS * cap, pl.net[3].prec, pl.net[3].ws, pl.net[3].ws_bytes, stream));
+  B200_PROPAGATE(mlp_backward(descs[3], params + pl.net[3].p_off, pl.xat, pl.d_yat, grads + pl.net[3].p_off, pl.d_xat,
+                              (int64_t)SEG_ATLAS_ROWS * cap, pl.net[3].prec, pl.net[3].ws, pl.net[3].ws_bytes, stream, true));
   seg_chain_kernel<<<(unsigned)((2 * layer_rows + 255) / 256), 256, 0, st>>>(pl.d_xat, layer_rows, pl.d_uv1, pl.d_uv2);
   B200_CHECK_LAUNCH();
   for (int k = 2; k >= 0; --k)
-    B200_PROPAGATE(b200_mlp_backward(descs[k], params + pl.net[k].p_off, ins[k], douts[k], grads + pl.net[k].p_off, nullptr,
-                                     net_rows[k], pl.net[k].prec, pl.net[k].ws, pl.net[k].ws_bytes, stream));
+    B200_PROPAGATE(mlp_backward(descs[k], params + pl.net[k].p_off, ins[k], douts[k], grads + pl.net[k].p_off, nullptr,
+                                net_rows[k], pl.net[k].prec, pl.net[k].ws, pl.net[k].ws_bytes, stream, true));
   return B200_OK;
 }
 
@@ -422,10 +420,9 @@ int b200_mlp_pretrain_loss_grad(const B200MlpDesc* d, int32_t batch, float uv_ma
     set_error("workspace too small: need %lld bytes", (long long)(pl.bytes + 1024));
     return B200_ERR_WORKSPACE;
   }
-  PersistentWorkspaceScope persistent;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const int64_t total = b200_mlp_layout(d, nullptr, nullptr);
-  const int prec = (precision == B200_PREC_TC && b200_mlp_tc_architecture(d) > 0) ? B200_PREC_TC : B200_PREC_FP32;
+  const int prec = mlp_precision(d, precision);
   B200_CHECK_CUDA(cudaMemsetAsync(grads, 0, (size_t)total * 4, st));
   B200_CHECK_CUDA(cudaMemsetAsync(losses, 0, 4, st));
   const float t_norm = (float)((double)frame / ((double)T / 2.0) - 1.0);     // unwrap_utils.py:189
@@ -433,9 +430,9 @@ int b200_mlp_pretrain_loss_grad(const B200MlpDesc* d, int32_t batch, float uv_ma
   seg_pack_kernel<<<(unsigned)((pl.cap + 255) / 256), 256, 0, st>>>(reinterpret_cast<const float4*>(pl.x_map), pl.cap,
                                                                     pl.cap, pl.x3, nullptr);
   B200_CHECK_LAUNCH();
-  B200_PROPAGATE(b200_mlp_forward(d, params, pl.x3, pl.uv, pl.cap, 1, prec, pl.ws, pl.ws_bytes, stream));
+  B200_PROPAGATE(mlp_forward(d, params, pl.x3, pl.uv, pl.cap, 1, prec, pl.ws, pl.ws_bytes, stream, true));
   B200_PROPAGATE(launch_pretrain_loss(pl.x_map, pl.uv, batch, pl.cap, uv_mapping_scale, pl.d_uv, losses, pl.counters, st));
-  B200_PROPAGATE(b200_mlp_backward(d, params, pl.x3, pl.d_uv, grads, nullptr, pl.cap, prec, pl.ws, pl.ws_bytes, stream));
+  B200_PROPAGATE(mlp_backward(d, params, pl.x3, pl.d_uv, grads, nullptr, pl.cap, prec, pl.ws, pl.ws_bytes, stream, true));
   return B200_OK;
 }
 
@@ -490,12 +487,10 @@ int b200_seg_render(const B200SegConfig* cfg, const float* params, int32_t H, in
   }
   int64_t offs[4];
   B200_REQUIRE(b200_seg_param_floats(cfg, offs) > 0, "invalid network descriptor");
-  PersistentWorkspaceScope persistent;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const B200MlpDesc* descs[4] = {&cfg->mapping1, &cfg->mapping2, &cfg->alpha, &cfg->atlas};
   int prec[4];
-  for (int k = 0; k < 4; ++k)
-    prec[k] = (cfg->precision == B200_PREC_TC && b200_mlp_tc_architecture(descs[k]) > 0) ? B200_PREC_TC : B200_PREC_FP32;
+  for (int k = 0; k < 4; ++k) prec[k] = mlp_precision(descs[k], cfg->precision);
   const int larger = W > H ? W : H;
   const float t_norm = (float)((double)frame / ((double)T / 2.0) - 1.0);      // evaluate.py:311
   const int64_t rp = pl.rows_pad;
@@ -505,10 +500,10 @@ int b200_seg_render(const B200SegConfig* cfg, const float* params, int32_t H, in
   B200_CHECK_LAUNCH();
   float* const outs[3] = {pl.uv1, pl.uv2, pl.ar};
   for (int k = 0; k < 3; ++k)
-    B200_PROPAGATE(b200_mlp_forward(descs[k], params + offs[k], pl.x3, outs[k], rp, 0, prec[k], pl.ws, pl.ws_bytes, stream));
+    B200_PROPAGATE(mlp_forward(descs[k], params + offs[k], pl.x3, outs[k], rp, 0, prec[k], pl.ws, pl.ws_bytes, stream, true));
   seg_atlas_in_kernel<<<(unsigned)((2 * rp + 255) / 256), 256, 0, st>>>(pl.uv1, pl.uv2, rp, pl.xat);
   B200_CHECK_LAUNCH();
-  B200_PROPAGATE(b200_mlp_forward(descs[3], params + offs[3], pl.xat, pl.yat, 2 * rp, 0, prec[3], pl.ws, pl.ws_bytes, stream));
+  B200_PROPAGATE(mlp_forward(descs[3], params + offs[3], pl.xat, pl.yat, 2 * rp, 0, prec[3], pl.ws, pl.ws_bytes, stream, true));
   seg_compose_kernel<<<(unsigned)((count + 255) / 256), 256, 0, st>>>(pl.yat, pl.ar, count, rp, rgb, rgb_u8, alpha);
   B200_CHECK_LAUNCH();
   return B200_OK;

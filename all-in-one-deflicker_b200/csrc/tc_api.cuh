@@ -1,8 +1,18 @@
-// Interface between c_api.cu and the tcgen05 path (mlp_tc.cu).
+// Interface of the tcgen05 path (mlp_tc.cu) and of the network calls that choose between it and the fp32 path
+// (c_api.cu), used by c_api.cu, seg.cu and eval_maps.cu.
 #pragma once
 #include "common.cuh"
 
 namespace b200 {
+
+// The network shapes the tensor-core kernels are specialised to (hidden width 256 each); every other shape runs on the
+// fp32 kernels.  Mapping6 is the stage-1 scripts' mapping (3 -> 256 x 4 -> 2, no encoding, no skips), Mapping4 the
+// background mapping of the segmentation variant (same kernels, two hidden 256x256 layers), Atlas the atlas network
+// (2 -> PE 10 -> 256 x 6 -> 3, skips 4 and 7) and Alpha the alpha network of the segmentation variant (3 -> PE 5 ->
+// 256 x 6 -> 1, no skips).  Atlas and Alpha run the kernel variants with a positional-encoding input layer.
+enum class TcNet { None, Mapping6, Mapping4, Atlas, Alpha };
+TcNet tc_classify(const MlpShape& s);    // None: no tensor-core kernels for this shape
+inline bool tc_pe_kernels(TcNet n) { return n == TcNet::Atlas || n == TcNet::Alpha; }
 
 // Buffers of the tensor-core path, carved from the caller's workspace (see mlp_tc.cu).
 struct TcPlan {
@@ -38,23 +48,26 @@ int64_t tc_infer_workspace_bytes(const MlpShape& ms, const MlpShape& as);
 int tc_infer_forward(const MlpShape& ms, const MlpShape& as, const float* params, const float* x_map, float* uv,
                      float* y, int64_t rows, char* ws, cudaStream_t st);
 
-// stand-alone IMLP (one network, autograd): see mlp_tc.cu
-int64_t tc_single_workspace_bytes(const MlpShape& sh, bool is_atlas, int64_t rows);
+// stand-alone IMLP (one network of family `net`, autograd): see mlp_tc.cu
+int64_t tc_single_workspace_bytes(const MlpShape& sh, TcNet net, int64_t rows);
 // persistent: the caller keeps this workspace and these parameter / gradient buffers across calls -> job tables are
-// cached in their own device allocations and the calls become graph-capturable after one eager call
-int tc_single_forward(const MlpShape& sh, bool is_atlas, const float* params, const float* x, float* y, int64_t rows,
+// cached in their own device allocations and the calls become graph-capturable after one eager call; otherwise they
+// are uploaded into the workspace on every call
+int tc_single_forward(const MlpShape& sh, TcNet net, const float* params, const float* x, float* y, int64_t rows,
                       bool training, char* ws, bool persistent, cudaStream_t st);
-int tc_single_backward(const MlpShape& sh, bool is_atlas, const float* params, float* grads, const float* x,
+int tc_single_backward(const MlpShape& sh, TcNet net, const float* params, float* grads, const float* x,
                        const float* y, const float* dy, float* d_in, int* gmax2, int64_t rows, char* ws, bool persistent,
                        cudaStream_t st);
 
-// Scope guard used by entry points that own a persistent workspace (the segmentation step): while alive,
-// b200_mlp_forward / backward calls made by this thread use the cached-table path above.
-struct PersistentWorkspaceScope {
-  PersistentWorkspaceScope();
-  ~PersistentWorkspaceScope();
-  bool prev;
-};
+// b200_mlp_forward / b200_mlp_backward with the persistence of the tensor-core job tables chosen by the caller: true
+// only for callers that keep `ws`, `params` and the gradient buffer alive across calls (the entry points of seg.cu)
+int mlp_forward(const B200MlpDesc* d, const float* params, const float* x, float* y, int64_t rows, int training,
+                int precision, void* ws, int64_t ws_bytes, void* stream, bool persistent);
+int mlp_backward(const B200MlpDesc* d, const float* params, const float* x, const float* dy, float* dparams, float* dx,
+                 int64_t rows, int precision, void* ws, int64_t ws_bytes, void* stream, bool persistent);
+// B200_PREC_TC when `precision` asks for it and the network has tensor-core kernels, else B200_PREC_FP32: for callers
+// that run each of several networks at the best precision it has
+int mlp_precision(const B200MlpDesc* d, int precision);
 
 int tc_debug_wgrad(long long* cycles, int* shapes, int max_ctas);
 

@@ -44,6 +44,30 @@ def test_invalid_descriptor_is_rejected_with_message():
     assert b"invalid" in N.lib().b200_last_error()
 
 
+def test_tc_architecture_accepts_exactly_the_stage1_shapes():
+    """b200_mlp_tc_architecture: 1 for the mapping (6 or 4 layers), 2 atlas, 3 alpha; a shape one attribute away from
+    one of them has no tensor-core kernels (0); an invalid descriptor is -1."""
+    def arch(in_dim, out_dim, hidden, layers, pe, skips):
+        d = N.MlpDesc(in_dim, out_dim, hidden, layers, pe, sum(1 << l for l in skips), 1, 0)
+        return N.lib().b200_mlp_tc_architecture(C.byref(d))
+    mapping6, mapping4 = (3, 2, 256, 6, 0, ()), (3, 2, 256, 4, 0, ())
+    atlas, alpha = (2, 3, 256, 8, 10, (4, 7)), (3, 1, 256, 8, 5, ())
+    assert [arch(*s) for s in (mapping6, mapping4, atlas, alpha)] == [1, 1, 2, 3]
+    near_misses = [
+        (3, 2, 256, 5, 0, ()), (3, 2, 256, 7, 0, ()),                 # layers
+        (2, 3, 256, 7, 10, (4,)), (2, 3, 256, 9, 10, (4, 7)), (3, 1, 256, 7, 5, ()), (3, 1, 256, 9, 5, ()),
+        (3, 2, 128, 6, 0, ()), (3, 2, 128, 4, 0, ()), (2, 3, 128, 8, 10, (4, 7)), (3, 1, 128, 8, 5, ()),   # hidden
+        (2, 3, 256, 8, 9, (4, 7)), (3, 1, 256, 8, 4, ()), (3, 2, 256, 6, 4, ()),                          # pe
+        (2, 2, 256, 6, 0, ()), (3, 3, 256, 6, 0, ()), (3, 3, 256, 8, 10, (4, 7)), (2, 2, 256, 8, 10, (4, 7)),
+        (2, 1, 256, 8, 5, ()), (3, 2, 256, 8, 5, ()),                                                    # widths
+        (2, 3, 256, 8, 10, (4,)), (2, 3, 256, 8, 10, (7,)),           # atlas with one of its two skips
+        (2, 3, 256, 8, 10, (2, 4, 7)), (3, 1, 256, 8, 5, (4,)),       # an extra skip
+        (3, 2, 256, 6, 0, (3,)), (3, 2, 256, 4, 0, (2,)),             # a mapping with a skip
+    ]
+    assert [arch(*s) for s in near_misses] == [0] * len(near_misses)
+    assert arch(3, 2, 256, 1, 0, ()) == -1
+
+
 def test_workspace_sizes_are_positive_and_monotone():
     lib = N.lib()
     small = N.AtlasConfig(1000, 1, N.PREC_FP32, 768, 0.8, 1, 100, 5000, 1000, 1, 5, 500)
